@@ -10,6 +10,9 @@
   ... --impl baseline     the library arm (baseline/torch_library_arm.py: cuBLASLt + SDPA + DDP + fused multi-tensor AdamW;
                           for tp: NCCL collectives + separate GEMMs) — none of the repo's kernels for gpt2 / resnet50
   ... --impl reference    the TF-1.15 reference: not installable in this image, prints {"unavailable": ...}
+  ... --dump-outputs DIR  after the timed steps, save the last one's loss and a fixed sample of the updated parameters as .npy
+                          (same arguments -> same inputs and, for one build, the same outputs, so two builds compare
+                          output for output)
 
 Metric/config follow BASELINE.json: GPT-2-XL (48 layers, d=1600, 25 heads), sequence 1024, bf16 compute with fp32 master
 weights, synthetic tokens, random-init weights, full training step (forward + backward + gradient reduction + AdamW)
@@ -51,7 +54,13 @@ def parse():
   ap.add_argument("--no-e2e", action="store_true")
   ap.add_argument("--no-graph", action="store_true", help="do not capture the training step in a CUDA graph")
   ap.add_argument("--profile", default="", help="write a per-kernel GPU time table of 2 extra steps to this file")
-  return ap.parse_args()
+  ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                  help="write what the last timed step returned on rank 0 (loss, sample of rank 0's updated parameters: its "
+                       "shard or stage under ZeRO-3 / tensor / pipeline parallelism) to DIR/<name>.npy")
+  args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  return args
 
 
 class ClockSampler(threading.Thread):
@@ -84,6 +93,36 @@ class ClockSampler(threading.Thread):
         reasons.append(name)
     smax = max((float(r[1]) for r in self.rows if len(r) > 1 and r[1].replace(".", "").isdigit()), default=0.0)
     return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": smax or None, "reasons": reasons, "samples": len(self.rows)}
+
+
+DUMP_PARAM_SAMPLE = 1 << 22          # 16 MB of float32: enough to see a wrong update, small enough to store and compare
+
+
+def dump_outputs(wl, loss, out_dir):
+  """What a caller of the timed step receives: its loss, and the model parameters it updated in place.
+
+  All parameters, flattened and concatenated in ``named_parameters()`` order, are sampled at fixed positions (seeded, sorted),
+  so two builds run with the same arguments write arrays that compare element for element; a model smaller than the sample
+  is written whole."""
+  import numpy as np
+  import torch
+  model = wl.trainer.model if wl.trainer is not None else wl.lib.raw
+  params = [p.detach() for _, p in model.named_parameters()]
+  total = sum(p.numel() for p in params)
+  if total <= DUMP_PARAM_SAMPLE:
+    sample = torch.cat([p.reshape(-1).float().cpu() for p in params])
+  else:
+    idx = torch.randint(total, (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    parts, start = [], 0
+    for p in params:
+      lo, hi = torch.searchsorted(idx, torch.tensor([start, start + p.numel()])).tolist()
+      if hi > lo:
+        parts.append(p.reshape(-1)[(idx[lo:hi] - start).to(p.device)].float().cpu())
+      start += p.numel()
+    sample = torch.cat(parts)
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "loss.npy"), np.asarray(float(loss), dtype=np.float32))
+  np.save(os.path.join(out_dir, "parameters.npy"), sample.numpy())
 
 
 # ============================================================================================ workloads
@@ -377,6 +416,8 @@ def main():
         f.write(text)
     barrier()
   ms, loss, clocks, launches = timed(args.steps, False)
+  if args.dump_outputs and rank == 0:            # before the untimed steps below move the weights on
+    dump_outputs(wl, loss, args.dump_outputs)
   value = wl.units_per_step * args.steps / (ms / 1e3)
   graphed = trainer is not None and getattr(trainer, "_graphed", None) is not None and trainer._graphed.graph is not None
   if graphed and phase is not None:

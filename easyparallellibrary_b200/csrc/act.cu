@@ -60,8 +60,9 @@ __global__ void __launch_bounds__(256) gelu_bwd_kernel(const T* __restrict__ pre
   }
 }
 
-// column sums: scratch[d] += sum_r x[r][d].  Block (32, 8): thread x owns 16 bytes of consecutive columns, rows are
-// strided over threadIdx.y and blockIdx.y; per-CTA smem reduction, one fp32 atomicAdd per column per CTA.
+// column sums: scratch[blockIdx.y][d] = sum over this CTA's rows of x[r][d].  Block (32, 8): thread x owns 16 bytes of
+// consecutive columns, rows are strided over threadIdx.y and blockIdx.y; per-CTA smem reduction, one partial per column per
+// CTA row, summed in row order by finish_colsum_kernel (no atomics: the result does not depend on which CTA finishes first).
 template <typename T>
 __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ x, float* __restrict__ scratch, int rows, int D) {
   constexpr int E = 16 / sizeof(T);
@@ -95,17 +96,30 @@ __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ x, fl
 #pragma unroll
     for (int k = 0; k < 8; ++k) t += s[k][c];
     const int gc = blockIdx.x * 32 * E + c;
-    if (gc < D) atomicAdd(&scratch[gc], t);
+    if (gc < D) scratch[(size_t)blockIdx.y * D + gc] = t;
   }
 }
 
+// out[d] = sum over the partial rows of scratch[.][d] in a fixed order: block (32, 8), thread (x, y) adds rows y, y + 8, ...
+// of column x in row order, then the eight sums are added in y order.
 template <typename T>
-__global__ void finish_colsum_kernel(const float* __restrict__ scratch, T* __restrict__ out, int D, int accumulate) {
-  int d = blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void __launch_bounds__(256) finish_colsum_kernel(const float* __restrict__ scratch, T* __restrict__ out, int D, int parts,
+                                                            int accumulate) {
+  __shared__ float s[8][33];
+  const int d = blockIdx.x * 32 + threadIdx.x;
+  float v = 0.f;
   if (d < D) {
-    float v = scratch[d];
-    if (accumulate) v += to_f32<T>(out[d]);
-    out[d] = from_f32<T>(v);
+#pragma unroll 4
+    for (int y = threadIdx.y; y < parts; y += 8) v += scratch[(size_t)y * D + d];
+  }
+  s[threadIdx.y][threadIdx.x] = v;
+  __syncthreads();
+  if (threadIdx.y == 0 && d < D) {
+    float t = s[0][threadIdx.x];
+#pragma unroll
+    for (int k = 1; k < 8; ++k) t += s[k][threadIdx.x];
+    if (accumulate) t += to_f32<T>(out[d]);
+    out[d] = from_f32<T>(t);
   }
 }
 
@@ -154,16 +168,23 @@ extern "C" int epl_gelu_bwd(const void* pre, const void* dy, void* dpre, int64_t
   return EPL_CHECK_LAUNCH();
 }
 
-// scratch: D floats, zeroed by this call
+// CTA rows of the colsum grid = rows of fp32[D] partials the caller provides as scratch
+extern "C" int epl_colsum_parts(int rows, int D, int dtype) {
+  const int E = 16 / (dtype == 0 ? 4 : 2);
+  const int gx = (D + 32 * E - 1) / (32 * E);
+  return std::max(1, std::min((rows + 31) / 32, (8 * kNumSMs + gx - 1) / gx));
+}
+
+// scratch: fp32 [epl_colsum_parts(rows, D, dtype), D]
 extern "C" int epl_colsum(const void* x, void* out, void* scratch, int rows, int D, int dtype, int accumulate, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  cudaMemsetAsync(scratch, 0, (size_t)D * sizeof(float), st);
+  const int parts = epl_colsum_parts(rows, D, dtype);
   BY_DTYPE(dtype, {
     constexpr int E = 16 / sizeof(T);
     const int gx = (D + 32 * E - 1) / (32 * E);
-    dim3 block(32, 8), grid(gx, std::max(1, std::min((rows + 31) / 32, (8 * kNumSMs + gx - 1) / gx)));
+    dim3 block(32, 8), grid(gx, parts);
     colsum_kernel<T><<<grid, block, 0, st>>>((const T*)x, (float*)scratch, rows, D);
-    finish_colsum_kernel<T><<<(D + 255) / 256, 256, 0, st>>>((const float*)scratch, (T*)out, D, accumulate);
+    finish_colsum_kernel<T><<<(D + 31) / 32, dim3(32, 8), 0, st>>>((const float*)scratch, (T*)out, D, parts, accumulate);
   });
   return EPL_CHECK_LAUNCH();
 }

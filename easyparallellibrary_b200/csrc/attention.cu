@@ -15,7 +15,11 @@
 // Backward: one CTA per (128-key tile, head, batch) looping over the query tiles that see it.  Five GEMMs per tile pair
 // (S = Q K^T, dP = dO V^T, dV += P^T dO, dK += dS^T Q, dQ_t = dS K), all on tcgen05 with K-major or MN-major shared-
 // memory descriptors over the *same* TMA-loaded tiles; dV/dK accumulate in TMEM across the loop, dQ tiles are reduced
-// into an fp32 buffer with atomics and converted once at the end.
+// into fp32 buffers and summed once at the end.  Key tiles 2m and 2m+1 reduce into slot m of the buffer: a zeroed
+// accumulator that receives exactly two fp32 adds ends with the same bits in either arrival order, and the final sum runs
+// over the slots in a fixed order, so dQ is bitwise reproducible from run to run.  At most kDqGroupTiles key tiles run per
+// launch; longer sequences take several launches, each folding its slots into a running fp32 total in slot order, so the
+// scratch stays at most kDqGroupTiles / 2 + 1 dQ-sized fp32 buffers whatever the sequence length.
 //
 // The reference computes attention as unfused softmax(QK^T)V framework ops (examples/bert/modeling.py attention_layer).
 #include "epl_common.cuh"
@@ -115,7 +119,8 @@ struct AttnParams {
   float* lse;             // [B,H,S]  (natural-log units)
   // backward only
   const float* delta;     // [B,H,S]  rowsum(dO * O)
-  float* dq_acc;          // [B,S,H,64] fp32, zero on entry
+  float* dq_acc;          // [slots,B,S,H,64] fp32, slot (kt-kt0)/2 zero on entry where key tile kt adds to it
+  int kt0;                // first key tile of this launch (blockIdx.x = kt - kt0)
   __nv_bfloat16* dqkv;    // [B,S,3,H,64]
   long long* dbg;         // optional phase timestamps of CTA (0,0,0): [step][8] softmax warp 2, [64 + step][8] MMA thread
 };
@@ -366,17 +371,43 @@ __global__ void __launch_bounds__(256) attn_delta_kernel(const __nv_bfloat16* __
   }
 }
 
-// dq (bf16, inside dqkv) <- dq_acc (fp32) * 1 ; 8 elements per thread
-__global__ void __launch_bounds__(256) attn_dq_convert_kernel(const float* __restrict__ acc, __nv_bfloat16* __restrict__ dqkv,
-                                                               int64_t rows, int H) {
+// dQ of one launch (key tiles kt0 ..): v = (first launch ? 0 : total) + slots 0, 1, ... in slot order; written as bf16 into
+// dqkv after the last launch, else to the fp32 total.  8 elements per thread.  Causal: query tile i only received adds from
+// key tiles kt0 .. i, i.e. from slots <= (i - kt0) / 2.
+__global__ void __launch_bounds__(256) attn_dq_convert_kernel(const float* __restrict__ acc, float* __restrict__ dq_total,
+                                                               __nv_bfloat16* __restrict__ dqkv, int64_t rows, int H, int S,
+                                                               int causal, int slots, int kt0, int first, int last_launch) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;       // over rows * H * 8 chunks
   const int64_t total = rows * H * (kD / 8);
   if (i >= total) return;
   const int64_t row = i / (H * (kD / 8));
   const int rem = (int)(i % (H * (kD / 8)));
   const int hh = rem / (kD / 8), ch = rem % (kD / 8);
-  const float4 a = reinterpret_cast<const float4*>(acc + (row * H + hh) * kD + ch * 8)[0];
-  const float4 b2 = reinterpret_cast<const float4*>(acc + (row * H + hh) * kD + ch * 8)[1];
+  const int qt = (int)(row % S) / kTile;
+  const int last = !causal ? slots - 1 : (qt < kt0 ? -1 : min((qt - kt0) / 2, slots - 1));
+  const int64_t off = (row * H + hh) * kD + ch * 8;
+  const float* src = acc + off;
+  float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b2 = a;
+  int m = 0;
+  if (!first) {
+    a = reinterpret_cast<const float4*>(dq_total + off)[0];
+    b2 = reinterpret_cast<const float4*>(dq_total + off)[1];
+  } else if (last >= 0) {
+    a = reinterpret_cast<const float4*>(src)[0];
+    b2 = reinterpret_cast<const float4*>(src)[1];
+    m = 1;
+  }
+  for (; m <= last; ++m) {
+    const float4 x = reinterpret_cast<const float4*>(src + (int64_t)m * rows * H * kD)[0];
+    const float4 y = reinterpret_cast<const float4*>(src + (int64_t)m * rows * H * kD)[1];
+    a.x += x.x; a.y += x.y; a.z += x.z; a.w += x.w;
+    b2.x += y.x; b2.y += y.y; b2.z += y.z; b2.w += y.w;
+  }
+  if (!last_launch) {
+    reinterpret_cast<float4*>(dq_total + off)[0] = a;
+    reinterpret_cast<float4*>(dq_total + off)[1] = b2;
+    return;
+  }
   uint4 w;
   w.x = pack_bf16x2(a.x, a.y); w.y = pack_bf16x2(a.z, a.w); w.z = pack_bf16x2(b2.x, b2.y); w.w = pack_bf16x2(b2.z, b2.w);
   *reinterpret_cast<uint4*>(dqkv + (row * 3 * H + hh) * kD + ch * 8) = w;
@@ -445,10 +476,11 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_consta
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tiles = (p.S + kTile - 1) / kTile;
-  const int kt = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
+  const int kt = p.kt0 + blockIdx.x, h = blockIdx.y, b = blockIdx.z;
   const int k0 = kt * kTile;
   const int i_begin = p.causal ? kt : 0;
   const int n_q = tiles - i_begin;
+  const int dq_slot_b = (blockIdx.x >> 1) * p.B + b;  // dQ goes to slot (kt-kt0)/2 (outer coordinate of the map: slot * B + b)
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&map_qkv); tma_prefetch_desc(&map_do);
@@ -538,7 +570,7 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_consta
         // dQ tile of the previous iteration -> fp32 accumulation buffer (also frees P / dS for rewriting)
         mbar_wait(dq_full, (n - 1) & 1);
         tc_fence_after();
-        flush_dq_tile(smem + BwdSmem::kDQ, t_dq + lane_addr, r, half, issuer, p.scale, &map_dq, h * kD, (i - 1) * kTile, b);
+        flush_dq_tile(smem + BwdSmem::kDQ, t_dq + lane_addr, r, half, issuer, p.scale, &map_dq, h * kD, (i - 1) * kTile, dq_slot_b);
       }
 #pragma unroll 1
       for (int ch = 0; ch < 2; ++ch) {
@@ -574,7 +606,8 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_consta
     {
       mbar_wait(dq_full, (n_q - 1) & 1);
       tc_fence_after();
-      flush_dq_tile(smem + BwdSmem::kDQ, t_dq + lane_addr, r, half, issuer, p.scale, &map_dq, h * kD, (i_begin + n_q - 1) * kTile, b);
+      flush_dq_tile(smem + BwdSmem::kDQ, t_dq + lane_addr, r, half, issuer, p.scale, &map_dq, h * kD, (i_begin + n_q - 1) * kTile,
+                    dq_slot_b);
     }
     if (issuer) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // all dQ reductions have landed
     // dK, dV of this key tile -> dqkv (row = key index): half 0 writes dV (slot 2), half 1 writes dK (slot 1)
@@ -679,7 +712,14 @@ extern "C" int epl_attn_fwd(const void* qkv, void* out, void* lse, int B, int S,
   return EPL_CHECK_LAUNCH();
 }
 
-// dq_acc: fp32 [B,S,H,64] scratch (zeroed here); delta: fp32 [B,H,S] scratch
+// dq_acc: fp32 [epl_attn_dq_slots(S),B,S,H,64] scratch (zeroed here where it is added to); delta: fp32 [B,H,S] scratch.
+// One launch: ceil(tiles / 2) slots; several launches: kDqGroupTiles / 2 slots + the running total.
+constexpr int kDqGroupTiles = 16;
+extern "C" int epl_attn_dq_slots(int S) {
+  const int tiles = (S + kTile - 1) / kTile;
+  return tiles <= kDqGroupTiles ? (tiles + 1) / 2 : kDqGroupTiles / 2 + 1;
+}
+
 extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out, const void* lse, void* delta, void* dq_acc,
                             void* dqkv, int B, int S, int H, float scale, int causal, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
@@ -688,7 +728,9 @@ extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out,
   if (rc) return rc;
   rc = make_map_3d(&map_do, d_out, B, S, (uint64_t)H * kD);
   if (rc) return rc;
-  rc = make_map_3d_f32(&map_dq, dq_acc, B, S, (uint64_t)H * kD);
+  const int tiles = (S + kTile - 1) / kTile;
+  const int slots = std::min((tiles + 1) / 2, kDqGroupTiles / 2);       // per launch; slot index `slots` holds the total
+  rc = make_map_3d_f32(&map_dq, dq_acc, (uint64_t)slots * B, S, (uint64_t)H * kD);
   if (rc) return rc;
   static bool configured = false;
   if (!configured) {
@@ -698,13 +740,24 @@ extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out,
   }
   const int64_t rows = (int64_t)B * S * H;
   attn_delta_kernel<<<(int)((rows + 127) / 128), 256, 0, st>>>((const __nv_bfloat16*)out, (const __nv_bfloat16*)d_out, (float*)delta, B, S, H);
-  cudaMemsetAsync(dq_acc, 0, (size_t)rows * kD * sizeof(float), st);
+  const size_t row_bytes = (size_t)H * kD * sizeof(float);
+  float* dq_total = (float*)dq_acc + (size_t)slots * B * S * H * kD;
+  const int64_t chunks = (int64_t)B * S * H * (kD / 8);
   AttnParams p{};
   p.B = B; p.S = S; p.H = H; p.scale = scale; p.causal = causal; p.lse = (float*)const_cast<void*>(lse);
   p.delta = (const float*)delta; p.dq_acc = (float*)dq_acc; p.dqkv = (__nv_bfloat16*)dqkv;
-  dim3 grid((S + kTile - 1) / kTile, H, B);
-  attn_bwd_kernel<<<grid, kBwdThreads, BwdSmem::kTotal, st>>>(map_qkv, map_do, map_dq, p);
-  const int64_t chunks = (int64_t)B * S * H * (kD / 8);
-  attn_dq_convert_kernel<<<(int)((chunks + 255) / 256), 256, 0, st>>>((const float*)dq_acc, (__nv_bfloat16*)dqkv, (int64_t)B * S, H);
+  for (int kt0 = 0; kt0 < tiles; kt0 += kDqGroupTiles) {
+    const int n_kt = std::min(kDqGroupTiles, tiles - kt0);
+    for (int m = 0; m < (n_kt + 1) / 2; ++m) {         // causal: slot m is added to from query tile kt0 + 2m on
+      const int r0 = causal ? std::min((kt0 + 2 * m) * kTile, S) : 0;
+      char* base = (char*)dq_acc + ((size_t)m * B * S + r0) * row_bytes;
+      if (r0 < S) cudaMemset2DAsync(base, (size_t)S * row_bytes, 0, (size_t)(S - r0) * row_bytes, B, st);
+    }
+    p.kt0 = kt0;
+    attn_bwd_kernel<<<dim3(n_kt, H, B), kBwdThreads, BwdSmem::kTotal, st>>>(map_qkv, map_do, map_dq, p);
+    attn_dq_convert_kernel<<<(int)((chunks + 255) / 256), 256, 0, st>>>((const float*)dq_acc, dq_total, (__nv_bfloat16*)dqkv,
+                                                                         (int64_t)B * S, H, S, causal, (n_kt + 1) / 2, kt0,
+                                                                         kt0 == 0, kt0 + kDqGroupTiles >= tiles);
+  }
   return EPL_CHECK_LAUNCH();
 }

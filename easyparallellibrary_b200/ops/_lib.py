@@ -64,6 +64,7 @@ class _Sigs:
   epl_bias_gelu_fwd = [_p, _p, _p, _p, _l, _i, _i, _p]
   epl_gelu_bwd = [_p, _p, _p, _l, _i, _p]
   epl_colsum = [_p, _p, _p, _i, _i, _i, _i, _p]
+  epl_colsum_parts = [_i, _i, _i]
   epl_add = [_p, _p, _p, _l, _i, _p]
   epl_xent = [_p, _p, _p, _p, _p, _p, _i, _i, _i, _f, _l, _i, _i, _i, _p]
   epl_scale_by_device_scalar = [_p, _p, _l, _i, _p]

@@ -22,6 +22,7 @@ def _lib_attn():
     p, i, f = ctypes.c_void_p, ctypes.c_int, ctypes.c_float
     lib.epl_attn_fwd.argtypes = [p, p, p, i, i, i, f, i, p]
     lib.epl_attn_bwd.argtypes = [p, p, p, p, p, p, p, i, i, i, f, i, p]
+    lib.epl_attn_dq_slots.argtypes = [i]
     _ready[0] = True
   return lib
 
@@ -53,7 +54,7 @@ class _FlashPacked(torch.autograd.Function):
     d_out = d_out.contiguous()
     dqkv = torch.empty_like(qkv)
     delta = torch.empty((B, H, S), dtype=torch.float32, device=qkv.device)
-    dq_acc = torch.empty((B, S, H, D), dtype=torch.float32, device=qkv.device)
+    dq_acc = torch.empty((lib.epl_attn_dq_slots(S), B, S, H, D), dtype=torch.float32, device=qkv.device)  # see csrc/attention.cu
     rc = lib.epl_attn_bwd(qkv.data_ptr(), out.data_ptr(), d_out.data_ptr(), lse.data_ptr(), delta.data_ptr(), dq_acc.data_ptr(),
                           dqkv.data_ptr(), B, S, H, ctx.scale, int(ctx.causal), _lib.stream())
     _lib.check(rc, "attn_bwd")

@@ -74,7 +74,7 @@ def colsum(x2: torch.Tensor) -> torch.Tensor:
   lib = _lib.require()
   rows, D = x2.shape
   out = torch.empty(D, dtype=x2.dtype, device=x2.device)
-  scratch = torch.empty(D, dtype=torch.float32, device=x2.device)
+  scratch = torch.empty(lib.epl_colsum_parts(rows, D, _lib.dtype_code(x2.dtype)), D, dtype=torch.float32, device=x2.device)
   rc = lib.epl_colsum(x2.data_ptr(), out.data_ptr(), scratch.data_ptr(), rows, D, _lib.dtype_code(x2.dtype), 0, _lib.stream())
   _lib.check(rc, "colsum")
   _lib.launches += 1

@@ -52,8 +52,8 @@ def fix_randomness(seed: int = 0, deterministic: bool = True) -> None:
   two runs to 1e-5 / 1e-6 (``tests/test_utils.py:25-33``: seeds + ``TF_DETERMINISTIC_OPS``).  Call it before building the model.
 
   The in-tree kernels are deterministic for a fixed launch configuration except where partial results meet in memory in arrival
-  order: the dQ accumulation of the attention backward (TMA reduce-add over key tiles) and bf16 weight-gradient accumulation
-  across micro-batches; runs then agree to rounding, not bit for bit."""
+  order: bf16 weight-gradient accumulation across micro-batches; runs then agree to rounding, not bit for bit.  (The dQ
+  accumulation of the attention backward and the bias-gradient column sums are reproducible bit for bit.)"""
   import os
   import random
   import numpy as np

@@ -51,8 +51,18 @@ def _run_once(fn, world, args, env, timeout):
   q = ctx.Queue()
   port = _free_port()
   procs = [ctx.Process(target=_entry, args=(r, world, port, fn, args, q, env)) for r in range(world)]
-  for p in procs:
-    p.start()
+  # the workers inherit the environment at start: with no visible GPU the library takes its CPU path (gloo, CPU tensors) on any
+  # machine, instead of placing every rank on the same device of a one-GPU box
+  visible = os.environ.get("CUDA_VISIBLE_DEVICES")
+  os.environ["CUDA_VISIBLE_DEVICES"] = ""
+  try:
+    for p in procs:
+      p.start()
+  finally:
+    if visible is None:
+      del os.environ["CUDA_VISIBLE_DEVICES"]
+    else:
+      os.environ["CUDA_VISIBLE_DEVICES"] = visible
   results = {}
   try:
     for _ in range(world):

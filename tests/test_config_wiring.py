@@ -210,10 +210,15 @@ def test_check_gradients_flag_validates_recompute():
 
 
 # ------------------------------------------------------------------------------------------------ cluster.run_visible_devices
-def test_run_visible_devices_is_exported_before_cuda_starts(monkeypatch):
-  monkeypatch.delenv("CUDA_VISIBLE_DEVICES", raising=False)
-  epl.init(epl.Config({"cluster.run_visible_devices": "2,3"}), init_process_group=False)
-  if torch.cuda.is_available() and torch.cuda.is_initialized():
-    pytest.skip("CUDA context already exists in this process")
-  assert os.environ.get("CUDA_VISIBLE_DEVICES") == "2,3"
-  monkeypatch.delenv("CUDA_VISIBLE_DEVICES", raising=False)
+def test_run_visible_devices_is_exported_before_cuda_starts():
+  """Checked in a fresh interpreter: on a machine with a GPU, earlier tests of this process have already started CUDA."""
+  import subprocess
+  import sys
+  root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+  code = ("import os\nimport easyparallellibrary_b200 as epl\n"
+          "epl.init(epl.Config({'cluster.run_visible_devices': '2,3'}), init_process_group=False)\n"
+          "print(os.environ.get('CUDA_VISIBLE_DEVICES'))\n")
+  env = {k: v for k, v in os.environ.items() if k != "CUDA_VISIBLE_DEVICES"}
+  env["PYTHONPATH"] = root + os.pathsep + env.get("PYTHONPATH", "")
+  r = subprocess.run([sys.executable, "-c", code], cwd=root, env=env, capture_output=True, text=True, timeout=300)
+  assert r.returncode == 0 and r.stdout.split()[-1:] == ["2,3"], r.stdout[-2000:] + r.stderr[-2000:]

@@ -252,7 +252,7 @@ def test_layernorm_fork_and_residual_linear():
 
 
 @pytest.mark.parametrize("causal", [True, False])
-@pytest.mark.parametrize("B,S,H", [(2, 256, 3), (1, 1024, 2), (2, 200, 2), (1, 384, 4)])
+@pytest.mark.parametrize("B,S,H", [(2, 256, 3), (1, 1024, 2), (2, 200, 2), (1, 384, 4), (1, 4160, 2)])  # 4160: 3 launches
 def test_flash_attention_packed(B, S, H, causal):
   """tcgen05 flash attention fwd + bwd vs fp32 softmax(QK^T)V autograd."""
   from easyparallellibrary_b200.ops.attention_kernel import flash_attention_packed
@@ -273,6 +273,27 @@ def test_flash_attention_packed(B, S, H, causal):
   g, gr = qkv.grad.float(), ref_in.grad
   for idx, name in enumerate(("dq", "dk", "dv")):
     _close(g[:, :, idx], gr[:, :, idx], 3e-2, 3e-2 * gr[:, :, idx].abs().max().item(), "attn " + name)
+
+
+@pytest.mark.parametrize("causal", [True, False])
+def test_backward_gradients_are_bitwise_reproducible(causal):
+  """Same inputs, same bits: the attention backward's dQ (slot-ordered sums, in one launch and in several) and the bias-gradient
+  column sums (partial rows added in a fixed order) do not depend on which CTA finishes first."""
+  from easyparallellibrary_b200.ops.attention_kernel import flash_attention_packed
+  from easyparallellibrary_b200.ops.linear import colsum
+  torch.manual_seed(0)
+  for B, S, H in ((8, 1024, 4), (1, 4160, 2)):
+    qkv = (torch.randn(B, S, 3, H, 64, device=DEV) * 0.8).bfloat16()
+    dout = torch.randn(B, S, H * 64, device=DEV).bfloat16()
+    grads = []
+    for _ in range(3):
+      x = qkv.clone().requires_grad_()
+      flash_attention_packed(x, causal).backward(dout)
+      grads.append(x.grad)
+    assert all(torch.equal(grads[0], g) for g in grads[1:]), (B, S, H)
+  x = torch.randn(8192, 1600, device=DEV).bfloat16()
+  sums = [colsum(x) for _ in range(3)]
+  assert all(torch.equal(sums[0], t) for t in sums[1:])
 
 
 @pytest.mark.parametrize("causal", [True, False])

@@ -298,14 +298,16 @@ def test_launcher_runs_a_two_process_job(tmp_path, amp):
     ("resnet/resnet_dp.py", ["--width", "8", "--classes", "32", "--image", "32", "--batch", "4", "--steps", "2", "--gc", "auto"]),
     ("resnet/resnet_split.py", ["--width", "8", "--classes", "32", "--image", "32", "--batch", "4", "--steps", "2"]),
     ("bert/run_squad.py", ["--model", "tiny", "--do_train", "--do_predict", "--num_train_steps", "3", "--train_batch_size", "4", "--synthetic_paragraphs", "8",
-                           "--output_dir", "/tmp/epl_squad_pytest_auto", "--auto_parallel", "--num_pipe_stages", "2", "--num_micro_batch", "2"]),
+                           "--auto_parallel", "--num_pipe_stages", "2", "--num_micro_batch", "2"]),
     ("bert/run_squad.py", ["--model", "tiny", "--do_train", "--do_predict", "--num_train_steps", "3", "--train_batch_size", "4",
-                           "--synthetic_paragraphs", "8", "--output_dir", "/tmp/epl_squad_pytest"]),
+                           "--synthetic_paragraphs", "8"]),
 ])
-def test_example_scripts_run_on_cpu(script, argv):
+def test_example_scripts_run_on_cpu(script, argv, tmp_path):
   """The examples (reference: examples/{bert,resnet,moe}) stay runnable: two steps of a tiny configuration on one CPU process."""
   import subprocess
   import sys
+  if script == "bert/run_squad.py":                  # its corpus, features and checkpoint go to a directory of this test only
+    argv = argv + ["--output_dir", str(tmp_path)]
   root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
   env = dict(os.environ, PYTHONPATH=root + os.pathsep + os.environ.get("PYTHONPATH", ""), CUDA_VISIBLE_DEVICES="")
   for k in ("RANK", "WORLD_SIZE", "LOCAL_RANK", "TF_CONFIG"):
@@ -485,7 +487,7 @@ def test_weight_ema_hook_with_clipping():
     out = tr.step(X[i], Y[i])
     assert out.grad_norm is not None
     d = min(0.1, (1.0 + i) / (10.0 + i))
-    expect = d * expect + (1 - d) * p0.detach()
+    expect = d * expect.to(p0.device) + (1 - d) * p0.detach()      # the trainer moved the model to its device in step 1
   name = ema._names[0]
   assert torch.allclose(ema.shadow[name], expect, atol=1e-7) and ema.updates == 4
   trained = p0.detach().clone()
