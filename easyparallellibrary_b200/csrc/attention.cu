@@ -123,7 +123,16 @@ struct AttnParams {
   int kt0;                // first key tile of this launch (blockIdx.x = kt - kt0)
   __nv_bfloat16* dqkv;    // [B,S,3,H,64]
   long long* dbg;         // optional phase timestamps of CTA (0,0,0): [step][8] softmax warp 2, [64 + step][8] MMA thread
+  const int* kv_len;      // optional device int32 [B]: batch row b sees keys [0, kv_len[b]) only (key padding), see key_len()
 };
+
+// Valid keys of batch row b.  Lengths are read on the device only (no host sync; a CUDA graph replays with whatever the buffer
+// holds) and clamped to [1, S], so a bad length cannot address outside the sequence and every query row keeps a key.  Keys at
+// or past the length are never loaded (forward) or contribute exact zeros (backward); their Q/K/V rows may hold any FINITE
+// values: the P V and dS^T Q products multiply the masked zeros by them, and 0 * Inf would be NaN.
+EPL_DEVICE int key_len(const AttnParams& p, int b) {
+  return p.kv_len ? min(max(p.kv_len[b], 1), p.S) : p.S;
+}
 
 // ================================================================================================================
 // forward
@@ -159,7 +168,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const AttnParams p)
   const int qt = q_tiles - 1 - (int)blockIdx.x;          // heaviest (causal) tiles first
   const int h = blockIdx.y, b = blockIdx.z;
   const int q0 = qt * kTile;
-  const int n_kv = p.causal ? qt + 1 : q_tiles;
+  const int len = key_len(p, b);
+  const int n_kv = min(p.causal ? qt + 1 : q_tiles, (len + kTile - 1) / kTile);   // key tiles past the length are skipped
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&map_qkv);
@@ -241,9 +251,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const AttnParams p)
       tmem_ld_32x32(my_s, v0);
       tmem_ld_32x32(my_s + 32, v1);
       const int k0 = j * kTile;
-      const bool need_mask = (k0 + kTile > p.S) || (p.causal && j == qt);
+      const bool need_mask = (k0 + kTile > len) || (p.causal && j == qt);
       // columns [0, lim) of this thread's half are visible to this query row (branch-free: one compare + select each)
-      const int lim = (need_mask ? min(p.S - k0, p.causal ? qidx - k0 + 1 : kTile) : kTile) - half * 64;
+      const int lim = (need_mask ? min(len - k0, p.causal ? qidx - k0 + 1 : kTile) : kTile) - half * 64;
       tmem_ld_wait();
       if (stamp) p.dbg[j * 8 + 2] = clock64();
       float mx = need_mask ? attn_half_max<true>(v0, v1, lim) : attn_half_max<false>(v0, v1, lim);
@@ -373,7 +383,8 @@ __global__ void __launch_bounds__(256) attn_delta_kernel(const __nv_bfloat16* __
 
 // dQ of one launch (key tiles kt0 ..): v = (first launch ? 0 : total) + slots 0, 1, ... in slot order; written as bf16 into
 // dqkv after the last launch, else to the fp32 total.  8 elements per thread.  Causal: query tile i only received adds from
-// key tiles kt0 .. i, i.e. from slots <= (i - kt0) / 2.
+// key tiles kt0 .. i, i.e. from slots <= (i - kt0) / 2.  With key lengths, a key tile past the length adds nothing: its slot
+// holds the memset zero plus zero or one add, exact either way, so neither this sum nor the memsets change.
 __global__ void __launch_bounds__(256) attn_dq_convert_kernel(const float* __restrict__ acc, float* __restrict__ dq_total,
                                                                __nv_bfloat16* __restrict__ dqkv, int64_t rows, int H, int S,
                                                                int causal, int slots, int kt0, int first, int last_launch) {
@@ -481,6 +492,19 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_consta
   const int i_begin = p.causal ? kt : 0;
   const int n_q = tiles - i_begin;
   const int dq_slot_b = (blockIdx.x >> 1) * p.B + b;  // dQ goes to slot (kt-kt0)/2 (outer coordinate of the map: slot * B + b)
+  const int len = key_len(p, b);
+
+  if (k0 >= len) {
+    // Key tile entirely past the length: its dK / dV are zero and it adds nothing to dQ (the slot it shares keeps the zero of
+    // the host memset plus at most the other tile's add, so dQ stays bitwise reproducible).  Every warp leaves here, before
+    // any barrier is initialised or TMEM allocated.
+    for (int i = threadIdx.x; i < kTile * 16; i += kBwdThreads) {     // [128 rows][dK, dV][8 16-byte chunks]
+      const int kidx = k0 + (i >> 4), which = 1 + ((i >> 3) & 1), ch = i & 7;
+      if (kidx < p.S)
+        *reinterpret_cast<uint4*>(p.dqkv + ((((size_t)b * p.S + kidx) * 3 + which) * p.H + h) * kD + ch * 8) = make_uint4(0, 0, 0, 0);
+    }
+    return;
+  }
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&map_qkv); tma_prefetch_desc(&map_do);
@@ -561,9 +585,9 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_consta
       const bool q_ok = qidx < p.S;
       const float lse2 = q_ok ? p.lse[((size_t)b * p.H + h) * p.S + qidx] * kLog2e : 0.f;
       const float dlt = q_ok ? p.delta[((size_t)b * p.H + h) * p.S + qidx] : 0.f;
-      const bool need_mask = (k0 + kTile > p.S) || (p.causal && i == kt) || !q_ok;
+      const bool need_mask = (k0 + kTile > len) || (p.causal && i == kt) || !q_ok;
       // columns [0, lim) of this thread's 64-column half are visible to this query row
-      const int lim0 = (!q_ok ? 0 : (need_mask ? min(p.S - k0, p.causal ? qidx - k0 + 1 : kTile) : kTile)) - half * 64;
+      const int lim0 = (!q_ok ? 0 : (need_mask ? min(len - k0, p.causal ? qidx - k0 + 1 : kTile) : kTile)) - half * 64;
       mbar_wait(sdp_full, n & 1);
       tc_fence_after();
       if (n > 0) {
@@ -695,7 +719,10 @@ using namespace epl;
 static long long* g_attn_dbg = nullptr;
 extern "C" void epl_attn_set_debug(void* ptr) { g_attn_dbg = (long long*)ptr; }
 
-extern "C" int epl_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int H, float scale, int causal, void* stream) {
+// kv_len: nullptr, or a device int32 [B] of key lengths (key_len() above).  Without it the kernels compute exactly what they
+// computed before lengths existed; so do lengths that are all S.
+extern "C" int epl_attn_fwd_len(const void* qkv, void* out, void* lse, int B, int S, int H, float scale, int causal, void* stream,
+                                const void* kv_len) {
   CUtensorMap map;
   int rc = make_map_3d(&map, qkv, B, S, (uint64_t)3 * H * kD);
   if (rc) return rc;
@@ -707,9 +734,14 @@ extern "C" int epl_attn_fwd(const void* qkv, void* out, void* lse, int B, int S,
   }
   AttnParams p{};
   p.B = B; p.S = S; p.H = H; p.scale = scale; p.causal = causal; p.out = (__nv_bfloat16*)out; p.lse = (float*)lse; p.dbg = g_attn_dbg;
+  p.kv_len = (const int*)kv_len;
   dim3 grid((S + kTile - 1) / kTile, H, B);
   attn_fwd_kernel<<<grid, kFwdThreads, FwdSmem::kTotal, (cudaStream_t)stream>>>(map, p);
   return EPL_CHECK_LAUNCH();
+}
+
+extern "C" int epl_attn_fwd(const void* qkv, void* out, void* lse, int B, int S, int H, float scale, int causal, void* stream) {
+  return epl_attn_fwd_len(qkv, out, lse, B, S, H, scale, causal, stream, nullptr);
 }
 
 // dq_acc: fp32 [epl_attn_dq_slots(S),B,S,H,64] scratch (zeroed here where it is added to); delta: fp32 [B,H,S] scratch.
@@ -720,8 +752,8 @@ extern "C" int epl_attn_dq_slots(int S) {
   return tiles <= kDqGroupTiles ? (tiles + 1) / 2 : kDqGroupTiles / 2 + 1;
 }
 
-extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out, const void* lse, void* delta, void* dq_acc,
-                            void* dqkv, int B, int S, int H, float scale, int causal, void* stream) {
+extern "C" int epl_attn_bwd_len(const void* qkv, const void* out, const void* d_out, const void* lse, void* delta, void* dq_acc,
+                                void* dqkv, int B, int S, int H, float scale, int causal, void* stream, const void* kv_len) {
   cudaStream_t st = (cudaStream_t)stream;
   CUtensorMap map_qkv, map_do, map_dq;
   int rc = make_map_3d(&map_qkv, qkv, B, S, (uint64_t)3 * H * kD);
@@ -745,7 +777,7 @@ extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out,
   const int64_t chunks = (int64_t)B * S * H * (kD / 8);
   AttnParams p{};
   p.B = B; p.S = S; p.H = H; p.scale = scale; p.causal = causal; p.lse = (float*)const_cast<void*>(lse);
-  p.delta = (const float*)delta; p.dq_acc = (float*)dq_acc; p.dqkv = (__nv_bfloat16*)dqkv;
+  p.delta = (const float*)delta; p.dq_acc = (float*)dq_acc; p.dqkv = (__nv_bfloat16*)dqkv; p.kv_len = (const int*)kv_len;
   for (int kt0 = 0; kt0 < tiles; kt0 += kDqGroupTiles) {
     const int n_kt = std::min(kDqGroupTiles, tiles - kt0);
     for (int m = 0; m < (n_kt + 1) / 2; ++m) {         // causal: slot m is added to from query tile kt0 + 2m on
@@ -760,4 +792,9 @@ extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out,
                                                                          kt0 == 0, kt0 + kDqGroupTiles >= tiles);
   }
   return EPL_CHECK_LAUNCH();
+}
+
+extern "C" int epl_attn_bwd(const void* qkv, const void* out, const void* d_out, const void* lse, void* delta, void* dq_acc,
+                            void* dqkv, int B, int S, int H, float scale, int causal, void* stream) {
+  return epl_attn_bwd_len(qkv, out, d_out, lse, delta, dq_acc, dqkv, B, S, H, scale, causal, stream, nullptr);
 }

@@ -6,6 +6,13 @@ Post-LN transformer encoder + a span-classification (SQuAD) head.  ``tensor_para
 attention and MLP from column/row-parallel pairs with token-sharded activations in between, i.e. the
 all-gather->GEMM and GEMM->reduce-scatter fused kernels carry all TP traffic.  ``num_pipeline_stages`` cuts the
 layer stack with ``epl.set_default_strategy`` exactly like ``examples/bert/modeling.py:829-834``.
+
+Model input: either token ids ``[B, S]`` (every position is a real token, segment 0 everywhere), or the SQuAD features
+``[B, 3, S]`` = ``stack(input_ids, input_mask, segment_ids)`` along dim 1.  ``input_mask`` must be right-padded (ones, then
+zeros), as every BERT feature pipeline produces it: attention sees it as a key length per sequence, ``input_mask.sum(-1)``, so
+padded keys are masked while padded query rows are still computed (their outputs are ignored by the loss).  The features travel
+as ONE tensor, so ``loss_fn(out, start, end)``, ``eval_step(features)`` and micro-batch splitting treat them like the ids.
+Layers after the embeddings read the mask from ``epl.current_micro_batch()[0]``.
 """
 from __future__ import annotations
 
@@ -45,6 +52,24 @@ class BertConfig:
     return 3.0 * L * (8 * d * d + 4 * d * f + 4 * seq_len * d)
 
 
+def split_features(features: torch.Tensor):
+  """``[B, S]`` ids -> ``(ids, None, None)``; ``[B, 3, S]`` features -> ``(input_ids, input_mask, segment_ids)``."""
+  if features.dim() == 3:
+    if features.shape[1] != 3:
+      raise ValueError("BERT features must be [B, S] ids or [B, 3, S] (input_ids, input_mask, segment_ids), got %s"
+                       % (tuple(features.shape),))
+    return features[:, 0], features[:, 1], features[:, 2]
+  return features, None, None
+
+
+def sequence_and_key_lengths():
+  """``(S, kv_len)`` of the micro-batch being executed: ``kv_len`` is the int32 ``[B]`` count of ones in the (right-padded)
+  ``input_mask``, or ``None`` for plain ``[B, S]`` ids (no padding)."""
+  import easyparallellibrary_b200 as epl
+  ids, mask, _ = split_features(epl.current_micro_batch()[0])
+  return ids.shape[1], (None if mask is None else mask.sum(-1, dtype=torch.int32))
+
+
 class BertEmbeddings(nn.Module):
   def __init__(self, cfg: BertConfig):
     super().__init__()
@@ -55,9 +80,12 @@ class BertEmbeddings(nn.Module):
     for e in (self.word, self.pos, self.typ):
       nn.init.normal_(e.weight, std=0.02)
 
-  def forward(self, ids):
+  def forward(self, features):
+    ids, _, seg = split_features(features)
     pos = torch.arange(ids.shape[1], device=ids.device)
-    return self.ln(self.word(ids) + self.pos(pos) + self.typ.weight[0])
+    if seg is None:
+      return self.ln(self.word(ids) + self.pos(pos) + self.typ.weight[0])
+    return self.ln(self.word(ids) + self.pos(pos) + self.typ(seg))
 
 
 class BertLayer(nn.Module):
@@ -76,7 +104,8 @@ class BertLayer(nn.Module):
     B, S, d = x.shape
     from easyparallellibrary_b200.ops.attention import attention_packed
     from easyparallellibrary_b200.ops.linear import linear
-    a = attention_packed(self.qkv(x).view(B, S, 3, self.heads, d // self.heads), causal=False)
+    _, kv_len = sequence_and_key_lengths()
+    a = attention_packed(self.qkv(x).view(B, S, 3, self.heads, d // self.heads), causal=False, kv_len=kv_len)
     x = self.ln1(linear(a, self.proj.weight, self.proj.bias, residual=x))
     return self.ln2(mlp(x, self.fc.weight, self.fc.bias, self.out.weight, self.out.bias, residual=x))
 
@@ -101,14 +130,13 @@ class BertLayerTP(nn.Module):
     self.seq_len = None
 
   def forward(self, x_shard):                      # [T/N, d]
-    S = self.seq_len
-    if S is None:                                  # a later pipeline stage: the sequence length comes from the micro-batch
-      import easyparallellibrary_b200 as epl
-      S = epl.current_micro_batch()[0].shape[1]
+    S, kv_len = sequence_and_key_lengths()         # token shards carry no sequence shape: it comes from the micro-batch
+    if self.seq_len is not None:
+      S = self.seq_len
     qkv = self.qkv(x_shard)                        # [T, 3d/N]  (all-gather -> GEMM)
-    T = qkv.shape[0]
+    T = qkv.shape[0]                               # the TP group's whole batch: T // S sequences, one length each
     from easyparallellibrary_b200.ops.attention import attention_packed
-    a = attention_packed(qkv.view(T // S, S, 3, self.heads_local, self.head_dim), causal=False).reshape(T, -1)
+    a = attention_packed(qkv.view(T // S, S, 3, self.heads_local, self.head_dim), causal=False, kv_len=kv_len).reshape(T, -1)
     x_shard = self.ln1(x_shard + self.proj(a))     # GEMM -> reduce-scatter
     return self.ln2(x_shard + self.out(self.fc(x_shard)))
 
@@ -136,13 +164,11 @@ class _TokenGather(nn.Module):
     self.split = split
 
   def forward(self, x):
-    import easyparallellibrary_b200 as epl
     from easyparallellibrary_b200.ops.tensor_parallel import current_tp_group
     g = current_tp_group(self.split)
-    ids = epl.current_micro_batch()[0]
-    B, S = ids.shape[0], ids.shape[1]
+    S, _ = sequence_and_key_lengths()
     full = _gather_tokens(x, g) if x.requires_grad else g.comm.allgather(x)
-    return full.view(B, S, -1)
+    return full.view(-1, S, full.shape[-1])
 
 
 class SquadHead(nn.Module):
@@ -188,12 +214,14 @@ class Bert(nn.Module):
     tp_out = [self.gather] if self.gather is not None else []
     return [self.embed] + tp_in + list(self.layers) + tp_out + [self.head]
 
-  def forward(self, ids, start=None, end=None):
+  def forward(self, features, start=None, end=None):
+    """``features``: ``[B, S]`` token ids or ``[B, 3, S]`` (input_ids, input_mask, segment_ids), see the module docstring."""
     import easyparallellibrary_b200 as epl
     from easyparallellibrary_b200.ir.graph import Graph
-    if epl.current_micro_batch() is None:                   # called outside a Trainer step (plain module use)
-      Graph.get().current_micro_batch = (ids, start, end)
-    x = ids
+    cur = epl.current_micro_batch()
+    if cur is None or cur[0] is not features:               # called outside a Trainer step (plain module use)
+      Graph.get().current_micro_batch = (features, start, end)
+    x = features
     for block in self.epl_sequential():
       x = block(x)
     if start is None:

@@ -154,17 +154,24 @@ class _GraphedStage(object):
 
   Unlike ``torch.cuda.make_graphed_callables`` nothing goes through autograd at replay time: the backward graph ends with the
   accumulation of every parameter gradient into the trainer's flat gradient buckets (weight-gradient GEMMs write there
-  directly, the other gradients are added by captured ``add_`` kernels), so an F or B instruction costs the host one small
-  copy and one graph launch — no per-parameter AccumulateGrad nodes, hooks or Python per micro-batch."""
+  directly, the other gradients are added by captured ``add_`` kernels), so an F or B instruction costs the host a few small
+  copies and one graph launch — no per-parameter AccumulateGrad nodes, hooks or Python per micro-batch.
 
-  def __init__(self, fn, x, labels, pool):
+  Every stage keeps static copies of every tensor of the micro-batch, and the capture runs with ``current_micro_batch``
+  pointing at them: a layer that reads the micro-batch (BERT's attention reads its key lengths from the input mask) bakes
+  the static copy's address into the graph, and each replay first copies the micro-batch being executed into it."""
+
+  def __init__(self, fn, x, mb, last, pool):
     """Phase 1: capture the forward graph.  ALL forward graphs of a stage are captured before any backward graph, so that a
-    backward's temporaries can never be placed (by the shared pool) where another instance's saved activations live."""
+    backward's temporaries can never be placed (by the shared pool) where another instance's saved activations live.
+    ``mb``: static copies of the micro-batch; on stage 0 ``x`` is ``mb[0]``."""
     self.fn = fn
     self.x = x                                       # static input (requires_grad for stages > 0)
-    self.labels = tuple(labels)
+    self.mb = tuple(mb)
+    self.labels = self.mb[1:] if last else ()
     self.pool = pool
     self.g_fwd, self.g_bwd = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
+    Graph.get().current_micro_batch = self.mb
     with torch.cuda.graph(self.g_fwd, pool=pool):
       self.y = fn(self.x, *self.labels)              # keeps the autograd graph (and with it the saved activations) alive
     self.y_out = self.y.detach()
@@ -174,6 +181,7 @@ class _GraphedStage(object):
     params = [p for p in self.fn.parameters() if p.requires_grad]
     inputs = ([self.x] if self.x.requires_grad else []) + params
     self.gy = torch.ones_like(self.y) if ones_grad else torch.zeros_like(self.y)
+    Graph.get().current_micro_batch = self.mb
     with torch.cuda.graph(self.g_bwd, pool=self.pool):
       grads = torch.autograd.grad(outputs=(self.y,), inputs=tuple(inputs), grad_outputs=(self.gy,), allow_unused=True, retain_graph=True)
       k = 0
@@ -184,12 +192,12 @@ class _GraphedStage(object):
         if g is not None:
           grad_views[id(p)].add_(g.view_as(grad_views[id(p)]))
 
-  def forward(self, x, labels):
-    if x.data_ptr() != self.x.data_ptr():
+  def forward(self, x, mb):
+    for s, t in zip(self.mb, mb):
+      if isinstance(s, torch.Tensor) and s.data_ptr() != t.data_ptr():
+        s.copy_(t)
+    if self.x is not self.mb[0] and x.data_ptr() != self.x.data_ptr():
       self.x.detach().copy_(x)
-    for s, l in zip(self.labels, labels):
-      if s.data_ptr() != l.data_ptr():
-        s.copy_(l)
     self.g_fwd.replay()
     return self.y_out
 
@@ -272,10 +280,10 @@ class PipelineExecutor(object):
     fn = _StageFn(self.module, loss_fn, factor if self.last else 1.0, device=self.device)
     self.stage_fn = fn
     self.stage_factor = fn.factor
-    labels = tuple(t.clone() for t in mb[1:] if isinstance(t, torch.Tensor)) if self.last else ()
-    if self.last and len(labels) != len(mb) - 1:
+    if self.last and not all(isinstance(t, torch.Tensor) for t in mb[1:]):
       self.use_graphs = False
       return
+    labels = tuple(mb[1:]) if self.last else ()
     for p in self.module.parameters():           # captured weight-gradient GEMMs must accumulate (the buckets are zeroed per step)
       if hasattr(p, "epl_sink_fresh"):
         p.epl_sink_fresh = False
@@ -284,16 +292,18 @@ class PipelineExecutor(object):
     grad_views = {pid: v[0] for pid, v in tr._grad_view.items()}
 
     def make_x():
-      if self.first:
-        return mb[0].clone()
       x = torch.zeros(self._shape_fwd[0], dtype=self._shape_fwd[1], device=self.device)
       return x.requires_grad_() if x.is_floating_point() else x
+
+    def make_stage():
+      static_mb = tuple(t.clone() if isinstance(t, torch.Tensor) else t for t in mb)
+      return _GraphedStage(fn, static_mb[0] if self.first else make_x(), static_mb, self.last, pool)
     try:
       # one eager pass on a side stream first (torch's capture recipe), then k (forward, backward) graph pairs in one pool
       side = torch.cuda.Stream(device=self.device)
       side.wait_stream(torch.cuda.current_stream())
       with torch.cuda.stream(side):
-        xw = make_x()
+        xw = mb[0].clone() if self.first else make_x()
         yw = fn(xw, *labels)
         ins_w = ([xw] if xw.requires_grad else []) + [p for p in fn.parameters() if p.requires_grad]
         torch.autograd.grad((yw,), tuple(ins_w), (torch.ones_like(yw),), allow_unused=True)
@@ -301,7 +311,7 @@ class PipelineExecutor(object):
       torch.cuda.current_stream().wait_stream(side)
       torch.cuda.synchronize(self.device)
       pool = torch.cuda.graph_pool_handle()
-      self.graphed = [_GraphedStage(fn, make_x(), tuple(l.clone() for l in labels), pool) for _ in range(k)]
+      self.graphed = [make_stage() for _ in range(k)]
       for st in reversed(self.graphed):
         st.capture_backward(grad_views, ones_grad=self.last)
     except Exception as e:      # pragma: no cover - depends on the CUDA runtime
@@ -445,7 +455,7 @@ class PipelineExecutor(object):
         with phase_scope(ModelPhase.FORWARD):
           if use_graphs:
             st = self.graphed[ins.mb % len(self.graphed)]
-            y = st.forward(x, mb[1:] if self.last else ())
+            y = st.forward(x, mb)
             if self.last:
               losses.append(y / self.stage_factor if self.stage_factor != 1.0 else y.clone())
           else:
@@ -469,6 +479,8 @@ class PipelineExecutor(object):
         n_back += 1
         tr._last_micro_batch = n_back == self.M
         y = outputs.pop(ins.mb)
+        # a recomputed forward (gradient checkpointing) re-reads the micro-batch: it must be this one, not the last one run
+        graph.current_micro_batch = micro[ins.mb]
         if timing and self.last:                   # split the last stage's backward into host-issue and device time
           torch.cuda.current_stream().synchronize()    # (never a device-wide sync here: a posted NCCL receive would never drain)
           _tb0 = _time.perf_counter()

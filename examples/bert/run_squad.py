@@ -34,7 +34,7 @@ from easyparallellibrary_b200.utils.dataset import ShardedFileDataset
 
 # ------------------------------------------------------------------------------------------------ data
 SquadExample = collections.namedtuple("SquadExample", "qas_id question doc_tokens answer_text start_word end_word")
-Features = collections.namedtuple("Features", "unique_id example_index tokens token_to_word input_ids segment_ids start end")
+Features = collections.namedtuple("Features", "unique_id example_index tokens token_to_word input_ids input_mask segment_ids start end")
 
 
 def synthetic_squad(path: str, n_paragraphs: int, seed: int) -> str:
@@ -155,12 +155,18 @@ def convert_examples_to_features(examples, tok, max_seq_length, doc_stride, max_
         s_pos = e_pos = -1
       ids = tok.ids(tokens)
       pad = max_seq_length - len(ids)
-      feats.append(Features(uid, ei, tokens, t2w, ids + [0] * pad, seg + [0] * pad, s_pos, e_pos))
+      # input_mask: 1 for real tokens, 0 for padding (right-padded, as models/bert.py requires)
+      feats.append(Features(uid, ei, tokens, t2w, ids + [0] * pad, [1] * len(ids) + [0] * pad, seg + [0] * pad, s_pos, e_pos))
       uid += 1
       if start + length >= len(doc):
         break
       start += min(length, doc_stride)
   return feats
+
+
+def stack_features(chunk):
+  """The model input of a list of features: ``[N, 3, S]`` = (input_ids, input_mask, segment_ids), see models/bert.py."""
+  return torch.tensor([[f.input_ids, f.input_mask, f.segment_ids] for f in chunk])
 
 
 def write_feature_files(feats, directory, per_file):
@@ -170,16 +176,17 @@ def write_feature_files(feats, directory, per_file):
   for i in range(0, len(feats), per_file):
     path = os.path.join(directory, "features-%05d.pt" % (i // per_file))
     chunk = feats[i:i + per_file]
-    torch.save({"input_ids": torch.tensor([f.input_ids for f in chunk]), "start": torch.tensor([f.start for f in chunk]),
+    torch.save({"features": stack_features(chunk), "start": torch.tensor([f.start for f in chunk]),
                 "end": torch.tensor([f.end for f in chunk])}, path)
     files.append(path)
   return files
 
 
 def read_feature_file(path):
+  """Yields ``([3, S] features, start, end)`` per feature."""
   d = torch.load(path)
-  for i in range(d["input_ids"].shape[0]):
-    yield d["input_ids"][i], d["start"][i], d["end"][i]
+  for i in range(d["features"].shape[0]):
+    yield d["features"][i], d["start"][i], d["end"][i]
 
 
 # ------------------------------------------------------------------------------------------------ evaluation
@@ -203,8 +210,7 @@ def predict(trainer, examples, feats, batch_size, max_answer_length=30):
   best = {}
   for i in range(0, len(feats), batch_size):
     chunk = feats[i:i + batch_size]
-    ids = torch.tensor([f.input_ids for f in chunk])
-    logits = trainer.eval_step(ids)
+    logits = trainer.eval_step(stack_features(chunk))
     if logits is None:                                   # pipeline: only the last stage sees the logits
       continue
     logits = logits.float().cpu()
@@ -316,8 +322,8 @@ def main():
     while step < args.num_train_steps:
       ds.set_epoch(epoch)
       loader = torch.utils.data.DataLoader(ds, batch_size=batch, drop_last=True)
-      for ids, s, e in loader:
-        out = trainer.step(ids, s, e)
+      for features, s, e in loader:
+        out = trainer.step(features, s, e)
         if rank == 0 and (step % 10 == 0 or step < 3):
           print("step %d loss %.4f" % (step, float(out.loss)), flush=True)
         step += 1
